@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — Gaussians->voxels throughput of the splat hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A step is one forward pass of the splat op (pack + supertile lists + render; 3 kernel launches, replayed from a CUDA
 graph) over one synthetic sample of BASELINE.json configs[1]: `nuscenes_gs25600_solid.py` shape — 25 600 Gaussians
@@ -23,6 +23,10 @@ Keys follow the driver contract; see DESIGN.md "Measurement".
 `--impl reference` times that CPU port as the reference arm (the reference has no CPU implementation of the splat; its
 CUDA op cannot run without a GPU build of torch extensions — when oracle/_ref was shipped, its timing on this GPU is
 reported as `ref_cuda_op` in the main line).  It always runs on ONE host CPU (rank 0), whatever --gpus says.
+
+`--dump-outputs DIR` writes what the timed path returned in its last timed step (rank 0) as DIR/logits.npy, the
+[N, 18] float32 logits (46 MB).  The inputs are seeded, so two builds run with the same arguments can be compared
+output for output.
 """
 from __future__ import annotations
 
@@ -153,6 +157,14 @@ def _all_host_threads():
     return oracle.set_num_threads(n)
 
 
+def _dump_outputs(outdir, arrays):
+    """--dump-outputs: each array as <outdir>/<name>.npy, float32."""
+    import numpy as np
+    os.makedirs(outdir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(outdir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+
+
 def run_reference_arm(args):
     """Reference arm: the reference algorithm's CPU port on this box's host cores.  ONE host CPU at any --gpus:
     under torchrun rank 0 alone runs and prints it, the other ranks exit without work."""
@@ -164,8 +176,10 @@ def run_reference_arm(args):
     kw, inp, _ = make_splat_inputs(WORKLOAD, seed=0, perturb=args.perturb)
     for _ in range(min(max(args.warmup, 1), 3)):       # the port has no clocks or caches to warm beyond a few passes
         _cpu_port_once(kw, inp)
-    steps = max(1, args.steps)
+    steps = args.steps
     t = [_cpu_port_once(kw, inp) for _ in range(steps)]
+    if args.dump_outputs:
+        _dump_outputs(args.dump_outputs, {"logits": _LAST_PORT["logits"]})
     sec = sum(t) / len(t)
     value = G_COUNTED / sec
     sample = (f"{steps} full forward passes of the {WORKLOAD} sample (N=640000 points, G=25601), {sec:.3f} s each; "
@@ -189,7 +203,10 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="launch the three kernels of a step directly instead of replaying a CUDA graph")
     ap.add_argument("--perturb", action="store_true", help="jitter every point inside its voxel (LoadOccupancySurroundOcc(perturb=True)); "
                     "the shipped configs and BASELINE.md use exact voxel centres")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference_arm(args)
 
@@ -301,6 +318,8 @@ def main():
     sampler.start()
     total_ms = timed_region(K, step)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        _dump_outputs(args.dump_outputs, {"logits": outs[(K - 1) % N_SETS].cpu().numpy()})
     ms_per_step = total_ms / K
     value = world * G_COUNTED / (ms_per_step * 1e-3)
 

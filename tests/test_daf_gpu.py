@@ -66,8 +66,9 @@ def test_daf_matches_reference_golden():
     # both are fp32 atomically-accumulated sums: the slack is the golden's own measured distance from the fp64 oracle
     feat_t, shape_t, start_t = DAF.feature_maps_format(fms)
     r64 = oracle.daf_backward(feat_t.contiguous().numpy(), shape_t.numpy(), start_t.numpy(), loc.numpy(), w.numpy(), g.numpy(), "f64")
-    for name, mine, ref, truth in (("feat", gf, gold["grad_feat"], r64[0]), ("loc", gl, gold["grad_loc"], r64[1]),
-                                   ("w", gw, gold["grad_weights"], r64[2])):
+    rows = slice(None, None, int(gold["feat_row_stride"]))      # the golden keeps every stride-th feature row
+    for name, mine, ref, truth in (("feat", gf[:, :, rows], gold["grad_feat_rows"], r64[0][:, :, rows]),
+                                   ("loc", gl, gold["grad_loc"], r64[1]), ("w", gw, gold["grad_weights"], r64[2])):
         floor = float(np.abs(ref.astype(np.float64) - truth).max())
         err = np.abs(mine.cpu().numpy().astype(np.float64) - ref)
         tol = np.maximum(h.ATOL + h.RTOL * np.abs(ref), (h.K_FLOOR + 1.0) * floor)
