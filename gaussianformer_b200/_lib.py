@@ -27,7 +27,9 @@ EXPORTS = (
     "gf_splat_forward", "gf_splat_backward", "gf_splat_read_flags",
     "gf_daf_forward", "gf_daf_backward", "gf_daf_format", "gf_splat_ce_partials",
     "gf_daf_fused_supported", "gf_daf_fused_forward", "gf_daf_fused_backward",
+    "gf_occ_loss_workspace_bytes", "gf_occ_loss_forward",
 )
+GF_OCC_LABEL_OUT_OF_RANGE = 1
 
 
 class SplatDesc(Structure):
@@ -73,6 +75,12 @@ class DafFormatDesc(Structure):
                 ("hw", c_int32 * DAF_MAX_LEVELS)]
 
 
+class OccLossDesc(Structure):
+    _fields_ = [("B", c_int32), ("N", c_int32), ("C", c_int32), ("use_softmax", c_int32), ("ignore_index", c_int32),
+                ("lovasz_ignore", c_int32), ("ignore_empty", c_int32), ("empty_label", c_int32),
+                ("ce_weight", c_float), ("lovasz_weight", c_float), ("lovasz", c_int32)]
+
+
 class GfError(RuntimeError):
     pass
 
@@ -113,6 +121,9 @@ def lib():
         L.gf_daf_fused_forward.argtypes = [POINTER(DafFusedDesc)] + [c_void_p] * 10
         L.gf_daf_fused_backward.argtypes = [POINTER(DafFusedDesc)] + [c_void_p] * 14
         L.gf_daf_format.argtypes = [POINTER(DafFormatDesc), POINTER(c_void_p), c_void_p, c_int, c_void_p]
+        L.gf_occ_loss_workspace_bytes.restype = c_size_t
+        L.gf_occ_loss_workspace_bytes.argtypes = [POINTER(OccLossDesc)]
+        L.gf_occ_loss_forward.argtypes = [POINTER(OccLossDesc)] + [c_void_p] * 8 + [c_size_t, c_void_p]
         if L.gf_abi_version() != 2:
             raise ImportError("libgf_b200.so: ABI version mismatch")
         _lib = L

@@ -11,7 +11,7 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-SOURCES = ["cabi.cu", "splat_prep.cu", "splat_forward.cu", "splat_backward.cu", "splat_backward_bin.cu", "daf.cu", "daf_fused.cu", "daf_tma.cu"]
+SOURCES = ["cabi.cu", "splat_prep.cu", "splat_forward.cu", "splat_backward.cu", "splat_backward_bin.cu", "daf.cu", "daf_fused.cu", "daf_tma.cu", "occ_loss.cu"]
 LIB = os.path.join(HERE, "libgf_b200.so")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = [

@@ -56,6 +56,11 @@ int launch_daf_fused_backward(const gf_daf_desc &d, int K, const float *feat, co
                               const float *stats, const float *out, const float *grad_out, float *grad_feat,
                               float *grad_loc, float *grad_logits, int num_sms, cudaStream_t stream);
 
+int occ_loss_check(const gf_occ_loss_desc *d);
+size_t occ_loss_workspace_bytes(const gf_occ_loss_desc &d);
+int occ_loss_forward(const gf_occ_loss_desc &d, const float *pred, const uint8_t *labels, const uint8_t *mask,
+                     const float *weights, float *loss3, float *grad, uint32_t *status, void *ws, cudaStream_t stream);
+
 thread_local cudaEvent_t g_ev_before = nullptr, g_ev_after = nullptr;
 
 bool pdl_enabled() {
@@ -346,6 +351,28 @@ int gf_daf_format(const gf_daf_format_desc *desc, float *const *maps, float *tab
     for (int l = 0; l < desc->num_scale; ++l)
         GF_REQUIRE(aligned16(maps[l]), GF_ERR_INVALID_ARG, "daf format: map %d must be 16-byte aligned", l);
     return gf::launch_daf_format(*desc, maps, table, inverse != 0, static_cast<cudaStream_t>(stream_));
+}
+
+size_t gf_occ_loss_workspace_bytes(const gf_occ_loss_desc *desc) {
+    if (occ_loss_check(desc) != GF_OK) return 0;
+    return occ_loss_workspace_bytes(*desc);
+}
+
+int gf_occ_loss_forward(const gf_occ_loss_desc *desc, const float *pred, const uint8_t *labels, const uint8_t *mask,
+                        const float *class_weights, float *loss3, float *grad_pred, uint32_t *status, void *workspace,
+                        size_t workspace_bytes, gf_stream_t stream_) {
+    int rc = occ_loss_check(desc);
+    if (rc != GF_OK) return rc;
+    GF_REQUIRE(loss3 != nullptr, GF_ERR_INVALID_ARG, "occ_loss: loss3 is NULL");
+    if (static_cast<long long>(desc->B) * desc->N > 0)
+        GF_REQUIRE(pred && labels, GF_ERR_INVALID_ARG, "occ_loss: pred / labels is NULL");
+    const size_t need = occ_loss_workspace_bytes(*desc);
+    GF_REQUIRE(workspace != nullptr && workspace_bytes >= need, GF_ERR_WORKSPACE,
+               "occ_loss: workspace too small (%zu < %zu bytes)", workspace_bytes, need);
+    GF_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255u) == 0, GF_ERR_WORKSPACE,
+               "occ_loss: workspace must be 256-byte aligned");
+    return occ_loss_forward(*desc, pred, labels, mask, class_weights, loss3, grad_pred, status, workspace,
+                            static_cast<cudaStream_t>(stream_));
 }
 
 }  // extern "C"

@@ -235,3 +235,79 @@ def reference_fused_composition(daf_apply, feat, shape, start, loc, logits, poin
     weights = weights * (1 - all_miss.flatten(1, 2).float())
     features = daf_apply(feat, shape, start, loc, weights).reshape(B, A, K, -1)
     return features.sum(dim=2)
+
+
+OCC_LOSS_CASES = {
+    # name: (B, N, C, use_softmax)
+    "small": (2, 3001, 18, True),
+    "small_prob": (2, 3001, 18, False),
+    "cfg2": (1, 200 * 200 * 16, 18, True),            # config 2's grid, one sample
+    "cfg2_prob": (1, 200 * 200 * 16, 18, False),
+    "cfg5": (4, 200 * 200 * 16, 18, True),            # config 5: four samples per GPU
+}
+
+
+def make_occ_loss_inputs(name="small", seed=0, empty_label=17, empty_frac=0.8, overrides=None):
+    """Seeded CPU inputs of the occupancy loss shaped like ``GaussianHead`` hands them over: ``pred [B,C,N]`` (logits,
+    or probabilities for the ``*_prob`` cases), ``labels [B,N]`` int64 (about ``empty_frac`` of them ``empty_label``, the
+    rest uniform over the other classes), ``occ_mask = labels != 0`` (dataset/transform_3d.py:509) and class weights
+    drawn from [0.5, 1.3].  Logits are moderate (N(0, 1.5^2)), so Lovász errors are tie-free."""
+    B, N, C, use_softmax = OCC_LOSS_CASES[name]
+    if overrides:
+        B, N, C, use_softmax = (overrides.get(k, v) for k, v in zip(("B", "N", "C", "use_softmax"), (B, N, C, use_softmax)))
+    gen = torch.Generator().manual_seed(seed)
+    logits = torch.randn(B, C, N, generator=gen) * 1.5
+    pred = logits if use_softmax else torch.softmax(logits, dim=1)
+    other = torch.randint(0, C - 1, (B, N), generator=gen)
+    other = other + (other >= empty_label).long()                  # any class but the empty one
+    labels = torch.where(torch.rand(B, N, generator=gen) < empty_frac, torch.full_like(other, empty_label), other)
+    weights = 0.5 + 0.8 * torch.rand(C, generator=gen)
+    return dict(pred=pred.contiguous(), labels=labels, occ_mask=labels != 0, class_weights=weights,
+                use_softmax=use_softmax)
+
+
+def reference_occupancy_loss(pred, labels, occ_mask=None, class_weights=None, *, use_softmax=True, ce_weight=10.0,
+                             lovasz_weight=1.0, lovasz_ignore=17, ignore_empty=False, empty_label=17):
+    """The reference's composition in PyTorch, as ``OccupancyLoss.loss_voxel`` runs it for one prediction
+    (loss/occupancy_loss.py:102-149): boolean-mask selects of the labels and the logits, ``nn.CrossEntropyLoss`` or
+    ``nll_loss(log(clamp(p)))``, then the Lovász-softmax of loss/utils/lovasz_softmax.py:157-204 -- a loop over the
+    classes with one ``fg.sum() == 0`` host check and one ``torch.sort`` each.  Differentiable; the timing baseline of
+    tools/time_loss.py and the end-to-end comparison of the tests.  Returns (loss, ce part, lovasz part)."""
+    F = torch.nn.functional
+    if ignore_empty:
+        keep = labels != empty_label
+        occ_mask = keep if occ_mask is None else keep & occ_mask.flatten(1)
+    if occ_mask is not None:
+        occ_mask = occ_mask.flatten(1)
+        labels = labels[occ_mask][None]
+        pred = pred.transpose(1, 2)[occ_mask][None].transpose(1, 2)
+    labels = labels.long()
+    w = None if class_weights is None else class_weights.to(pred)
+    if use_softmax:
+        ce = F.cross_entropy(pred, labels, weight=w, ignore_index=255)
+        probas = torch.softmax(pred, dim=1)
+    else:
+        ce = F.nll_loss(torch.log(torch.clamp(pred, 1e-6, 1. - 1e-6)), labels, w, ignore_index=255)
+        probas = pred
+    probas = probas.transpose(1, 2).flatten(0, 1)
+    flat = labels.flatten()
+    if lovasz_ignore is not None:
+        keep = flat != lovasz_ignore
+        probas, flat = probas[keep], flat[keep]
+    losses = []
+    if probas.numel() > 0:
+        for c in range(probas.shape[1]):
+            fg = (flat == c).float()
+            if fg.sum() == 0:                                   # a host sync per class, as in the reference
+                continue
+            err = (fg - probas[:, c]).abs()
+            err_sorted, perm = torch.sort(err, 0, descending=True)
+            fg_sorted = fg[perm]
+            gts = fg_sorted.sum()
+            inter = gts - fg_sorted.cumsum(0)
+            union = gts + (1 - fg_sorted).cumsum(0)
+            jac = 1. - inter / union
+            jac = torch.cat([jac[:1], jac[1:] - jac[:-1]])
+            losses.append(torch.dot(err_sorted, jac))
+    lov = torch.stack(losses).mean() if losses else pred.new_zeros(())
+    return ce_weight * ce + lovasz_weight * lov, ce_weight * ce, lovasz_weight * lov

@@ -253,6 +253,47 @@ int gf_daf_fused_backward(const gf_daf_fused_desc *desc, const float *mc_ms_feat
                           float *grad_mc_ms_feat, float *grad_sampling_location, float *grad_weight_logits,
                           gf_stream_t stream);
 
+/* ---- occupancy loss: weighted cross-entropy + Lovász-softmax, value and gradient (no counterpart in the native
+ * reference: OccupancyLoss.loss_voxel, loss/occupancy_loss.py:102-149, with CE_ssc_loss :164-178 / CE_wo_softmax
+ * :180-183 and lovasz_softmax(classes='present', per_image=False), loss/utils/lovasz_softmax.py:157-204) ----
+ *
+ * All B*N points form ONE pooled set.  A point takes part when mask[i] != 0 (or mask == NULL) and, with ignore_empty,
+ * labels[i] != empty_label.  Of those:
+ *   CE      = sum w[y] nll / sum w[y] over y < C, y != ignore_index; nll = -log_softmax(pred)[y] (use_softmax) or
+ *             -log(clamp(pred[y], 1e-6, 1 - 1e-6)); NaN (0/0) when no point is left, as in torch
+ *   Lovász  = mean over the classes present in the set {y != lovasz_ignore} (255 labels stay in it as background) of
+ *             sum_i e_(i) dJ_i, e = |[y = c] - q_c| sorted in descending order, q = softmax(pred) or pred; 0 without a
+ *             present class.  Equal errors are ordered by point index (a stable sort; the reference leaves their order
+ *             to torch.sort).  dJ is computed in closed form from integer counts.  q is expected in [0, 1]; errors
+ *             above 1 are treated as 1
+ *   loss3   = [ce_weight * CE + lovasz_weight * Lovász, ce_weight * CE, lovasz_weight * Lovász]
+ *   grad    = d loss3[0] / d pred (torch's subgradients: abs'(0) = 0, clamp passes the gradient on [lo, hi]); 0 for
+ *             points that take no part
+ * Labels that are neither < C nor ignore_index contribute nothing and set GF_OCC_LABEL_OUT_OF_RANGE in *status.
+ * Loss and gradient are bit-identical between calls (fixed-order fp64 sums, no floating-point atomics). */
+#define GF_OCC_LABEL_OUT_OF_RANGE 1u
+
+typedef struct gf_occ_loss_desc {
+    int32_t B, N, C;        /* pred [B, N, C] row-major (the splat's logits layout); C in 16..20 */
+    int32_t use_softmax;    /* != 0: pred are logits (GaussianFormer-1); 0: probabilities (GaussianFormer-2) */
+    int32_t ignore_index;   /* CE ignore label, 0..255 (255 in the reference) */
+    int32_t lovasz_ignore;  /* label left out of the Lovász set, -1 = none (17 in the shipped configs) */
+    int32_t ignore_empty;   /* != 0: points labelled empty_label take no part */
+    int32_t empty_label;
+    float ce_weight;        /* loss_voxel_ce_weight */
+    float lovasz_weight;    /* loss_voxel_lovasz_weight */
+    int32_t lovasz;         /* != 0: compute the Lovász term (use_lovasz_loss) */
+} gf_occ_loss_desc;
+
+size_t gf_occ_loss_workspace_bytes(const gf_occ_loss_desc *desc);
+
+/* pred [B,N,C] fp32, labels [B,N] uint8, mask [B,N] uint8 or NULL, class_weights [C] or NULL (ones).  loss3 [3] and
+ * grad_pred [B,N,C] (NULL: no gradient) are fully overwritten, as is *status (device word, may be NULL).  The
+ * workspace needs no initialisation. */
+int gf_occ_loss_forward(const gf_occ_loss_desc *desc, const float *pred, const uint8_t *labels, const uint8_t *mask,
+                        const float *class_weights, float *loss3, float *grad_pred, uint32_t *status, void *workspace,
+                        size_t workspace_bytes, gf_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif
